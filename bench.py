@@ -2,6 +2,7 @@
 """Benchmark of the multi-view denoising hot path (BASELINE.json: "6-view 224x400 denoising-steps/sec").
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload full|cam] [--scenes S]
+                  [--dump-outputs DIR]
 
 One "step" = ControlNet forward + multi-view UNet forward + classifier-free-guidance combine + DDIM update for S
 six-view scenes per GPU (CFG on: 12 view-samples per scene-step, the reference default guidance_scale = 2).
@@ -32,7 +33,7 @@ TFLOP_PER_SCENE_STEP_CFG = {"224x400": 4.75, "424x800": 24.0}  # BASELINE.md sec
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=30)
+    ap.add_argument("--steps", type=int, default=30, help="timed denoising steps (>= 1)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="full", choices=["cam", "full"],
@@ -58,7 +59,31 @@ def parse():
     ap.add_argument("--strong-scaling", action="store_true",
                     help="N>1, default sharding: after the replica measurement also time ONE scene spread over all N GPUs "
                          "(guidance halves x views through NVLink peer memory) and report it as `strong_scaling`")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed loop's last step returned (the scene latents, float32) as DIR/<name>.npy, "
+                         "at most 64 MB in all, so that two builds can be compared output for output on identical inputs")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, arrays):
+    """Write each tensor of `arrays` as <dirname>/<name>.npy in float32.  When they exceed DUMP_LIMIT_BYTES in all, each is
+    replaced by the same share of its elements at positions drawn from a fixed seed, so that every run writes the same ones."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    total = sum(a.numel() for a in arrays.values()) * 4
+    for name, a in arrays.items():
+        a = a.detach().float().cpu()
+        if total > DUMP_LIMIT_BYTES:
+            flat = a.reshape(-1)
+            keep = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(0))[:flat.numel() * DUMP_LIMIT_BYTES // total]
+            a = flat[keep.sort().values]
+        np.save(os.path.join(dirname, name + ".npy"), a.numpy())
 
 
 def make_inputs(args, rank):
@@ -330,6 +355,8 @@ def main():
     barrier()
     clocks = sampler.stop()
     ms_total = e0.elapsed_time(e1)
+    # the latents a caller of the timed path receives after its last step; the sections below reuse and overwrite `st`
+    dumped = {"latents": pipe.latents_out(st)} if args.dump_outputs else None
     if world > 1:
         tt = torch.tensor([ms_total], device=dev)
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
@@ -563,6 +590,8 @@ def main():
         if strong is not None:
             line["strong_scaling"] = strong
         print(json.dumps(line))
+        if dumped is not None:
+            dump_outputs(args.dump_outputs, dumped)
     if world > 1:
         from magicdrive_b200.dist import shutdown
         sys.stdout.flush()

@@ -35,6 +35,23 @@ def test_reference_arm_prints_the_contract_line():
     assert cfg["sharding"].startswith("scene-per-GPU replicas") and cfg["scheduler"] == "ddim"
 
 
+def test_dump_outputs_caps_the_size_with_a_fixed_sample(tmp_path, monkeypatch):
+    """--dump-outputs: float32 .npy files; over the size limit, the same seeded sample of positions on every run."""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    x = torch.arange(1000, dtype=torch.float64).reshape(10, 100)
+    bench.dump_outputs(str(tmp_path / "full"), {"latents": x})
+    full = np.load(tmp_path / "full" / "latents.npy")
+    assert full.dtype == np.float32 and full.shape == (10, 100) and (full == x.numpy()).all()
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 400)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"latents": x})
+    a, b = np.load(tmp_path / "a" / "latents.npy"), np.load(tmp_path / "b" / "latents.npy")
+    assert a.nbytes <= 400 and a.size == 100 and (a == b).all()
+    assert (np.diff(a) > 0).all() and np.isin(a, full).all()
+
+
 @pytest.mark.skipif(torch.cuda.is_available(), reason="needs a machine WITHOUT a CUDA device")
 def test_our_arm_has_no_cpu_fallback():
     r = _run("--steps", "1", "--warmup", "1", timeout=300)
