@@ -57,6 +57,34 @@ def test_gemm_split_k(cuda_lib, splits):
     assert _rel(out, ref) < 2e-5, _rel(out, ref)
 
 
+@pytest.mark.parametrize("case", ["zero_conv", "conv3x3_shift"])
+def test_gemm_split_k_bf16_residual(cuda_lib, case):
+    """The planner's own split-K route (nothing forced) at the 4 x 7 level of the benchmark (V = 12, M = 336), bf16 output:
+    a ControlNet zero convolution onto the UNet skip (residual, out_scale) and a ResNet conv1 with its per-image time shift
+    (four images per M tile, which the pair kernel refuses) plus residual.  Every element within one bf16 rounding step."""
+    g = torch.Generator(device="cuda").manual_seed(15)
+    n, h, w, c = 12, 4, 7, 1280
+    x = _bf(torch.randn(n * h * w, c, device="cuda", generator=g))
+    r = _bf(torch.randn(n * h * w, c, device="cuda", generator=g))
+    b = torch.randn(c, device="cuda", generator=g)
+    n0 = ops.launch_count()
+    if case == "zero_conv":
+        wt = _bf(torch.randn(c, c, device="cuda", generator=g) / math.sqrt(c))
+        out = ops.linear(x, wt, bias=b, residual=r, out_scale=0.7)
+        ref = 0.7 * (x.float() @ wt.float().t() + b) + r.float()
+    else:
+        wt = _bf(torch.randn(c, c, 3, 3, device="cuda", generator=g) / math.sqrt(9 * c))
+        temb = torch.randn(n, c, device="cuda", generator=g)
+        out = ops.gemm_conv(x, _conv_weight(wt), n_img=n, h_in=h, w_in=w, c0=c, lda0=c, n_out=c, taps=3, pad=1, bias=b,
+                            rowbias=temb, residual=r, ldr=c)
+        xi = x.float().reshape(n, h, w, c).permute(0, 3, 1, 2)
+        ref = _nhwc(F.conv2d(xi, wt.float(), b, padding=1) + temb[:, :, None, None]) + r.float()
+    assert ops.launch_count() - n0 == 2  # split-K partials + finalize
+    err = (out.float() - ref).abs()
+    bad = (err > ref.abs() * 2.0 ** -7 + 2e-3 * ref.abs().max()).sum().item()
+    assert bad == 0, (bad, err.max().item())
+
+
 def test_gemm_strided_views(cuda_lib):
     """A read from a column slice of a wider buffer, output written into a column slice (fused-QKV style)."""
     g = torch.Generator(device="cuda").manual_seed(3)
