@@ -48,6 +48,9 @@ int mdb_device_ok(void);
  * GEGLU.proj + FeedForward out (attention.py:270,226), connector (magicdrive/networks/blocks.py:83),
  * ControlNet zero convs (magicdrive/networks/unet_addon_rawbox.py:221-272).
  * A may be split over two sources along channels (torch.cat skip connections, unet_2d_blocks.py:1984,2086).
+ * Taps that fall outside the input read zeros on every side, so h_out / w_out may exceed the symmetric-pad size: the VAE
+ * encoder's Downsample2D(padding=0) (resnet.py:215-220, F.pad(x, (0, 1, 0, 1)) then a stride-2 3x3 conv) is pad 0 with
+ * h_out = (h_in - 2) / 2 + 1 (w_out likewise).
  * ------------------------------------------------------------------------------------------------ */
 typedef struct {
   const void* a0;      /* bf16 [n_img, h_in, w_in, lda0] using the first c0 channels */
@@ -179,6 +182,21 @@ int mdb_bf16_to_f32(const void* x, float* out, long long n, void* stream);
  * that lets conv_in (unet_2d_condition.py:231, 4 -> 320 channels) run on the tensor-core path; repeat = 2 duplicates
  * the batch for classifier-free guidance (pipeline_bev_controlnet.py:352-354). */
 int mdb_pack_latents(const void* x, int x_is_f32, long long pix, int cin, int cpad, int repeat, void* out, void* stream);
+
+/* Image patches for the VAE encoder's conv_in (diffusers/models/vae.py:53-59, a 3x3 pad-1 nn.Conv2d from the cin = 3 image
+ * channels; called from AutoencoderKL.encode, autoencoder_kl.py:164): NCHW images [n, cin, h, w] (fp32 or bf16) ->
+ * bf16 [n*h*w, 64] where column (r*3 + s)*cin + c holds channel c at tap (r, s) of the zero-padded 3x3 neighbourhood and
+ * columns >= 9*cin are zero (cin <= 7).  conv_in then runs as one K = 64 GEMM on mdb_gemm_conv with its weight packed in
+ * the same column order, instead of a 9-tap conv over channels padded to 64.  out must be 16-byte aligned. */
+int mdb_pack_image_patches(const void* x, int x_is_f32, int n, int cin, int h, int w, void* out, void* stream);
+
+/* DiagonalGaussianDistribution of the encoder's moments (diffusers/models/vae.py:397-416; the demo's
+ * `vae.encode(x).latent_dist.mean * scaling_factor`, demo/run_cond_on_view.py:80-86): moments fp32 NHWC [n*h*w, ldm] with
+ * mean in columns [0, c) and logvar in [c, 2c) -> out fp32 NCHW [n, c, h, w] =
+ *   scale * (mean + exp(0.5 * clamp(logvar, -30, 20)) * noise)
+ * noise: fp32 NCHW [n, c, h, w] (the shape randn_tensor draws in) or NULL, which gives scale * mean. */
+int mdb_latent_dist(const float* moments, int ldm, int n, int c, int h, int w, const float* noise, float scale, float* out,
+                    void* stream);
 
 /* Classifier-free guidance + DDIM (eta = 0) update fused (pipeline_bev_controlnet.py:426-436;
  * scheduling_ddim.py:325-445).  eps: fp32 [(2 if cfg else 1) * n/c pixels, eps_ld] (uncond half first), c channels

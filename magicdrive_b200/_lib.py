@@ -61,6 +61,8 @@ SIGNATURES = {
     "mdb_f32_to_bf16": (_i, [_vp, _vp, _ll, _vp]),
     "mdb_bf16_to_f32": (_i, [_vp, _vp, _ll, _vp]),
     "mdb_pack_latents": (_i, [_vp, _i, _ll, _i, _i, _i, _vp, _vp]),
+    "mdb_pack_image_patches": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp]),
+    "mdb_latent_dist": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _f, _vp, _vp]),
     "mdb_cfg_ddim_step": (_i, [_vp, _i, _i, _i, _f, _vp, _vp, _ll, _vp]),
     "mdb_softmax_rows": (_i, [_vp, _i, _ll, _i, _vp, _i, _i, _vp]),
     "mdb_pin_views": (_i, [_vp, _i, _vp, _vp, _i, _vp, _vp, _ll, _i, _vp]),

@@ -351,34 +351,70 @@ def vae_decoder_blocks(cfg: VaeConfig):
     return blocks
 
 
+def _vae_resnet(sh, p, ci, co):
+    """ResnetBlock2D without a time embedding (resnet.py:525-589, temb_channels=None)."""
+    _norm(sh, p + ".norm1", ci)
+    _conv(sh, p + ".conv1", co, ci, 3)
+    _norm(sh, p + ".norm2", co)
+    _conv(sh, p + ".conv2", co, co, 3)
+    if ci != co:
+        _conv(sh, p + ".conv_shortcut", co, ci, 1)
+
+
+def _vae_mid_block(sh, p, c):
+    """UNetMidBlock2D of the VAE: single-head attention, then its two resnets (unet_2d_blocks.py:395-473)."""
+    a = p + ".attentions.0"
+    _norm(sh, a + ".group_norm", c)
+    for n in ("to_q", "to_k", "to_v", "to_out.0"):
+        _lin(sh, f"{a}.{n}", c, c)
+    _vae_resnet(sh, p + ".resnets.0", c, c)
+    _vae_resnet(sh, p + ".resnets.1", c, c)
+
+
 def vae_decoder_param_shapes(cfg: VaeConfig) -> "OrderedDict[str, tuple]":
     """Decoder + post_quant_conv keys of AutoencoderKL.state_dict() (vae.py:152-225, autoencoder_kl.py:107-108)."""
     sh: "OrderedDict[str, tuple]" = OrderedDict()
     c_mid = cfg.block_out_channels[-1]
     _conv(sh, "decoder.conv_in", c_mid, cfg.latent_channels, 3)
-
-    def res(p, ci, co):
-        _norm(sh, p + ".norm1", ci)
-        _conv(sh, p + ".conv1", co, ci, 3)
-        _norm(sh, p + ".norm2", co)
-        _conv(sh, p + ".conv2", co, co, 3)
-        if ci != co:
-            _conv(sh, p + ".conv_shortcut", co, ci, 1)
-
     for _, resnets, up in vae_decoder_blocks(cfg):
         for p, ci, co in resnets:
-            res(p, ci, co)
+            _vae_resnet(sh, p, ci, co)
         if up:
             _conv(sh, up, resnets[-1][2], resnets[-1][2], 3)
-    a = "decoder.mid_block.attentions.0"
-    _norm(sh, a + ".group_norm", c_mid)
-    for n in ("to_q", "to_k", "to_v", "to_out.0"):
-        _lin(sh, f"{a}.{n}", c_mid, c_mid)
-    res("decoder.mid_block.resnets.0", c_mid, c_mid)
-    res("decoder.mid_block.resnets.1", c_mid, c_mid)
+    _vae_mid_block(sh, "decoder.mid_block", c_mid)
     _norm(sh, "decoder.conv_norm_out", cfg.block_out_channels[0])
     _conv(sh, "decoder.conv_out", cfg.out_channels, cfg.block_out_channels[0], 3)
     _conv(sh, "post_quant_conv", cfg.latent_channels, cfg.latent_channels, 1)
+    return sh
+
+
+def vae_encoder_blocks(cfg: VaeConfig):
+    """[(prefix, [(resnet prefix, cin, cout)], downsampler conv prefix or None)] of Encoder.down_blocks: one
+    DownEncoderBlock2D per level with a padding-0 Downsample2D on every level but the last (vae.py:62-82,
+    unet_2d_blocks.py:1030-1087)."""
+    blocks, out_c = [], cfg.block_out_channels[0]
+    for i, c in enumerate(cfg.block_out_channels):
+        prev, out_c = out_c, c
+        res = [(f"encoder.down_blocks.{i}.resnets.{j}", prev if j == 0 else out_c, out_c) for j in range(cfg.layers_per_block)]
+        down = None if i == len(cfg.block_out_channels) - 1 else f"encoder.down_blocks.{i}.downsamplers.0.conv"
+        blocks.append((f"encoder.down_blocks.{i}", res, down))
+    return blocks
+
+
+def vae_encoder_param_shapes(cfg: VaeConfig) -> "OrderedDict[str, tuple]":
+    """Encoder + quant_conv keys of AutoencoderKL.state_dict() (vae.py:39-97 with double_z, autoencoder_kl.py:95-106)."""
+    sh: "OrderedDict[str, tuple]" = OrderedDict()
+    c_mid = cfg.block_out_channels[-1]
+    _conv(sh, "encoder.conv_in", cfg.block_out_channels[0], cfg.in_channels, 3)
+    for _, resnets, down in vae_encoder_blocks(cfg):
+        for p, ci, co in resnets:
+            _vae_resnet(sh, p, ci, co)
+        if down:
+            _conv(sh, down, resnets[-1][2], resnets[-1][2], 3)
+    _vae_mid_block(sh, "encoder.mid_block", c_mid)
+    _norm(sh, "encoder.conv_norm_out", c_mid)
+    _conv(sh, "encoder.conv_out", 2 * cfg.latent_channels, c_mid, 3)
+    _conv(sh, "quant_conv", 2 * cfg.latent_channels, 2 * cfg.latent_channels, 1)
     return sh
 
 

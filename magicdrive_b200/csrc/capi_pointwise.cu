@@ -327,6 +327,63 @@ __global__ void pack_latents_kernel(const TI* __restrict__ x, long long pix, int
   for (int r = 0; r < repeat; ++r) out[(r * pix + p) * cpad + c] = v;
 }
 
+// NCHW images [n, cin, h, w] (fp32 or bf16) -> bf16 [n*h*w, 64]: row = output pixel, column (r*3 + s)*cin + c = input
+// channel c at tap (r, s) of the zero-padded 3x3 neighbourhood, columns >= 9*cin zero.  The encoder's conv_in then runs
+// as one K = 64 GEMM.  A block stages a (TH + 2) x (TW + 2) halo tile of every channel in shared memory (each input
+// element is read from global memory once per tile) and writes each of its pixels as one 128-byte row: 8 threads x 16 bytes.
+constexpr int PATCH_TW = 32, PATCH_TH = 8, PATCH_MAXC = 7;
+template <typename TI>
+__global__ void __launch_bounds__(256) pack_image_patches_kernel(const TI* __restrict__ x, int cin, int h, int w,
+                                                                 uint4* __restrict__ out) {
+  __shared__ float tile[PATCH_MAXC][PATCH_TH + 2][PATCH_TW + 2];
+  const int img = blockIdx.z, y0 = blockIdx.y * PATCH_TH, x0 = blockIdx.x * PATCH_TW;
+  const TI* xi = x + static_cast<long long>(img) * cin * h * w;
+  constexpr int per_c = (PATCH_TH + 2) * (PATCH_TW + 2);
+  for (int i = threadIdx.x; i < cin * per_c; i += blockDim.x) {
+    const int c = i / per_c, rem = i - c * per_c;
+    const int r = rem / (PATCH_TW + 2), s = rem - r * (PATCH_TW + 2);
+    const int yy = y0 + r - 1, xx = x0 + s - 1;
+    tile[c][r][s] = (yy >= 0 && yy < h && xx >= 0 && xx < w) ? ldf(xi + (static_cast<long long>(c) * h + yy) * w + xx) : 0.f;
+  }
+  __syncthreads();
+  const int px = threadIdx.x >> 3, q = threadIdx.x & 7;  // pixel of the tile row, 16-byte chunk of its output row
+  const int xx = x0 + px;
+  if (xx >= w) return;
+  const int kcols = 9 * cin;
+  for (int r = 0; r < PATCH_TH && y0 + r < h; ++r) {
+    __align__(16) __nv_bfloat16 v[8];
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      const int col = q * 8 + j;
+      float f = 0.f;
+      if (col < kcols) {
+        const int tap = col / cin, c = col - tap * cin;
+        f = tile[c][r + tap / 3][px + tap % 3];
+      }
+      v[j] = __float2bfloat16_rn(f);
+    }
+    out[((static_cast<long long>(img) * h + y0 + r) * w + xx) * 8 + q] = *reinterpret_cast<const uint4*>(v);
+  }
+}
+
+// DiagonalGaussianDistribution of the encoder's moments: NHWC fp32 [pix, ldm] rows (mean[0:c] | logvar[c:2c]) -> NCHW fp32
+// [n, c, h, w] = scale * (mean + exp(0.5 * clamp(logvar, -30, 20)) * noise), noise NCHW like the output (null: scale * mean).
+__global__ void latent_dist_kernel(const float* __restrict__ mom, int ldm, int c, long long hw, long long total,
+                                   const float* __restrict__ noise, float scale, float* __restrict__ out) {
+  const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i >= total) return;
+  const long long nc = i / hw, p = i - nc * hw;
+  const long long img = nc / c;
+  const int ch = static_cast<int>(nc - img * c);
+  const float* m = mom + (img * hw + p) * ldm;
+  float v = m[ch];
+  if (noise) {
+    const float lv = fminf(fmaxf(m[c + ch], -30.f), 20.f);
+    v += expf(0.5f * lv) * noise[i];
+  }
+  out[i] = scale * v;
+}
+
 inline unsigned nblocks(long long n, int t) { return static_cast<unsigned>((n + t - 1) / t); }
 
 }  // namespace
@@ -467,6 +524,34 @@ extern "C" int mdb_pack_latents(const void* x, int x_is_f32, long long pix, int 
     pack_latents_kernel<__nv_bfloat16><<<nblocks(pix * cpad, 256), 256, 0, st>>>(
         static_cast<const __nv_bfloat16*>(x), pix, cin, cpad, repeat, static_cast<__nv_bfloat16*>(out));
   MDB_CHECK_LAUNCH("pack_latents_kernel");
+  return MDB_OK;
+}
+
+extern "C" int mdb_pack_image_patches(const void* x, int x_is_f32, int n, int cin, int h, int w, void* out, void* stream) {
+  if (!x || !out) return set_error(MDB_ERR_INVALID, "mdb_pack_image_patches: null pointer");
+  if (n <= 0 || h <= 0 || w <= 0 || cin < 1 || cin > PATCH_MAXC)
+    return set_error(MDB_ERR_INVALID, "mdb_pack_image_patches: bad shape (n=%d cin=%d h=%d w=%d; 9*cin must fit 64 columns)",
+                     n, cin, h, w);
+  if (reinterpret_cast<uintptr_t>(out) & 15) return set_error(MDB_ERR_INVALID, "mdb_pack_image_patches: out must be 16-byte aligned");
+  dim3 grid((w + PATCH_TW - 1) / PATCH_TW, (h + PATCH_TH - 1) / PATCH_TH, n);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (x_is_f32)
+    pack_image_patches_kernel<float><<<grid, 256, 0, st>>>(static_cast<const float*>(x), cin, h, w, static_cast<uint4*>(out));
+  else
+    pack_image_patches_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(static_cast<const __nv_bfloat16*>(x), cin, h, w,
+                                                                    static_cast<uint4*>(out));
+  MDB_CHECK_LAUNCH("pack_image_patches_kernel");
+  return MDB_OK;
+}
+
+extern "C" int mdb_latent_dist(const float* moments, int ldm, int n, int c, int h, int w, const float* noise, float scale,
+                               float* out, void* stream) {
+  if (!moments || !out) return set_error(MDB_ERR_INVALID, "mdb_latent_dist: null pointer");
+  if (n <= 0 || c <= 0 || h <= 0 || w <= 0 || ldm < 2 * c) return set_error(MDB_ERR_INVALID, "mdb_latent_dist: bad shape");
+  const long long hw = static_cast<long long>(h) * w, total = static_cast<long long>(n) * c * hw;
+  latent_dist_kernel<<<nblocks(total, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(moments, ldm, c, hw, total, noise,
+                                                                                         scale, out);
+  MDB_CHECK_LAUNCH("latent_dist_kernel");
   return MDB_OK;
 }
 

@@ -614,10 +614,10 @@ class VaeDecoderEngine:
                             residual=res, ldr=cout)
         return FMap(out, x.n, x.h, x.w, cout)
 
-    def _attention(self, x: FMap) -> FMap:
-        """Attention(heads=1, dim_head=C, GroupNorm, residual) of UNetMidBlock2D (unet_2d_blocks.py:433-446)."""
+    def _attention(self, x: FMap, a: str) -> FMap:
+        """Attention(heads=1, dim_head=C, GroupNorm, residual) of UNetMidBlock2D (unet_2d_blocks.py:433-446); `a` is its
+        key prefix (decoder.mid_block.attentions.0 or encoder.mid_block.attentions.0)."""
         W, C, L = self.W, x.c, x.h * x.w
-        a = "decoder.mid_block.attentions.0"
         g, b = W.norm(a + ".group_norm")
         t = ops.groupnorm(x.data, C, C, x.n, L, g, b, 1e-6, False, groups=self.cfg.norm_num_groups)
         wq, bq = W.lin(a + ".to_q")
@@ -627,7 +627,7 @@ class VaeDecoderEngine:
         lp = (L + 63) // 64 * 64  # keys padded to whole K blocks of the P.V product
         # persistent scratch (no per-call allocation or zero-fill: the decode is captured in a CUDA graph): scores and
         # probabilities [L, lp] per image, V^T [C, lp] whose pad columns stay zero from allocation (P is zero there too)
-        key = ("vae_attn", x.n, L, C)
+        key = ("vae_attn", a, x.n, L, C)
         if key not in W.t:
             dev = q.device
             # keys live in a buffer with lp - L spare rows so that every image's score GEMM can take lp "keys" (its n_out must
@@ -665,7 +665,7 @@ class VaeDecoderEngine:
         x = ops.conv_direct(x, wd, bd, n=n, h=h, w=w, cin=lc, cout=c, k=3)
         x = FMap(x.reshape(n * h * w, c), n, h, w, c)
         x = self._resnet("decoder.mid_block.resnets.0", x, c)
-        x = self._attention(x)
+        x = self._attention(x, "decoder.mid_block.attentions.0")
         x = self._resnet("decoder.mid_block.resnets.1", x, c)
         for _, resnets, up in self.blocks:
             for p, _, cout in resnets:
@@ -689,3 +689,79 @@ class VaeDecoderEngine:
                             bias=bo, out_f32=True, out_scale=0.5 if to_unit_range else 1.0)
         img = img.reshape(x.n, x.h, x.w, self.COUT_PAD)[..., : cfg.out_channels]
         return img.clamp(0, 1) if to_unit_range else img
+
+
+class VaeEncoderEngine(VaeDecoderEngine):
+    """AutoencoderKL.encode up to the moments (autoencoder_kl.py:160-171 -> Encoder.forward, vae.py:99-133, then
+    quant_conv).  It extends the decoder engine: the resnets, the single-head mid-block attention and the packed-weight
+    cache are the decoder's, so a module with both halves keeps one engine and can decode as well.
+      * conv_in (3 -> C0, 3x3) is one K = 64 GEMM over the image-patch matrix of mdb_pack_image_patches;
+      * Downsample2D(padding=0) (resnet.py:215-220) is the stride-2 implicit GEMM with pad 0 and h_out = (h - 2) // 2 + 1:
+        the F.pad(0, 1, 0, 1) row and column are the taps past the far edge, which read zeros;
+      * quant_conv (1x1, 8 -> 8) is folded into conv_out in fp32 (W' = W_q W_out per tap, b' = W_q b_out + b_q), whose fp32
+        epilogue writes the NHWC moments [pixels, 8] directly."""
+
+    PATCH_K = 64  # columns of the image-patch matrix: 27 taps x channels, zero-padded to one K block
+
+    def __init__(self, cfg: arch.VaeConfig, sd, device):
+        super().__init__(cfg, sd, device)
+        if 9 * cfg.in_channels > self.PATCH_K:
+            raise ValueError(f"VAE encoder: in_channels={cfg.in_channels} does not fit the {self.PATCH_K}-column patch matrix")
+        self.down = arch.vae_encoder_blocks(cfg)
+
+    def _conv_in_weight(self):
+        W = self.W
+        if "encoder.conv_in.wp" not in W.t:  # [C0, 3, 3, 3] -> [C0, 64], column (r*3 + s)*cin + c like the patch matrix
+            w = W.raw("encoder.conv_in.weight").float()
+            wp = torch.zeros((w.shape[0], self.PATCH_K), dtype=F32, device=w.device)
+            wp[:, : 9 * w.shape[1]] = w.permute(0, 2, 3, 1).reshape(w.shape[0], -1)
+            W.t["encoder.conv_in.wp"] = _bf(wp)
+            W.t["encoder.conv_in.b"] = _f32(W.raw("encoder.conv_in.bias"))
+        return W.t["encoder.conv_in.wp"], W.t["encoder.conv_in.b"]
+
+    @property
+    def moments_ld(self) -> int:
+        """Row stride of the moments: 2 * latent_channels rounded up to the GEMM's 8-column output granularity."""
+        return (2 * self.cfg.latent_channels + 7) // 8 * 8
+
+    def _conv_out_weight(self):
+        W = self.W
+        if "encoder.conv_out.wq" not in W.t:
+            wq = W.raw("quant_conv.weight").float()[:, :, 0, 0]  # [2c, 2c]
+            wo = W.raw("encoder.conv_out.weight").float()        # [2c, C, 3, 3]
+            m = wq.shape[0]
+            wf = torch.zeros((self.moments_ld, *wo.shape[1:]), dtype=F32, device=wo.device)
+            bf = torch.zeros((self.moments_ld,), dtype=F32, device=wo.device)
+            wf[:m] = torch.einsum("ij,jkrs->ikrs", wq, wo)
+            bf[:m] = wq @ W.raw("encoder.conv_out.bias").float() + W.raw("quant_conv.bias").float()
+            # pack_conv_weight's (tap, channel) K order, stored in fold_dtype like the other folded products
+            W.t["encoder.conv_out.wq"] = wf.permute(0, 2, 3, 1).reshape(wf.shape[0], -1).contiguous().to(W.fold_dtype)
+            W.t["encoder.conv_out.bq"] = bf
+        return W.t["encoder.conv_out.wq"], W.t["encoder.conv_out.bq"]
+
+    def encode(self, images: torch.Tensor) -> torch.Tensor:
+        """images: NCHW [n, in_channels, H, W] fp32 or bf16 (H, W divisible by 8) -> fp32 NHWC moments
+        [n * H/8 * W/8, moments_ld], columns [0, c) the mean and [c, 2c) the logvar before its clamp."""
+        cfg, W = self.cfg, self.W
+        n, _, h, w = images.shape
+        c0 = cfg.block_out_channels[0]
+        wi, bi = self._conv_in_weight()
+        xp = ops.pack_image_patches(images)
+        x = FMap(ops.linear(xp, wi, bias=bi), n, h, w, c0)
+        for _, resnets, down in self.down:
+            for p, _, cout in resnets:
+                x = self._resnet(p, x, cout)
+            if down:
+                wd, bd = W.conv(down)
+                ho, wo = (x.h - 2) // 2 + 1, (x.w - 2) // 2 + 1
+                out = ops.gemm_conv(x.data, wd, n_img=x.n, h_in=x.h, w_in=x.w, c0=x.c, lda0=x.c, n_out=x.c, taps=3, stride=2,
+                                    pad=0, h_out=ho, w_out=wo, bias=bd)
+                x = FMap(out, x.n, ho, wo, x.c)
+        x = self._resnet("encoder.mid_block.resnets.0", x, x.c)
+        x = self._attention(x, "encoder.mid_block.attentions.0")
+        x = self._resnet("encoder.mid_block.resnets.1", x, x.c)
+        g, b = W.norm("encoder.conv_norm_out")
+        hn = ops.groupnorm(x.data, x.c, x.c, x.n, x.h * x.w, g, b, 1e-6, True, groups=cfg.norm_num_groups)
+        wo_, bo = self._conv_out_weight()
+        return ops.gemm_conv(hn, wo_, n_img=x.n, h_in=x.h, w_in=x.w, c0=x.c, lda0=x.c, n_out=self.moments_ld, taps=3, pad=1,
+                             bias=bo, out_f32=True)

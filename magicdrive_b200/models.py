@@ -12,13 +12,13 @@ import logging
 import os
 from collections import OrderedDict
 from dataclasses import asdict, dataclass, fields
-from typing import Any, Dict, List, Tuple, Union
+from typing import Any, Dict, List, Optional, Tuple, Union
 
 import torch
 import torch.nn as nn
 
 from . import arch, ops
-from .engine import ControlNetEngine, UNetEngine, VaeDecoderEngine
+from .engine import ControlNetEngine, UNetEngine, VaeDecoderEngine, VaeEncoderEngine
 
 BF16, F32 = torch.bfloat16, torch.float32
 
@@ -114,7 +114,8 @@ class _B200Module(nn.Module):
             path = os.path.join(path, subfolder)
         with open(os.path.join(path, cls.config_name)) as f:
             raw = json.load(f)
-        model = cls(**{k: v for k, v in raw.items() if not k.startswith("_")})
+        # keyword arguments override / extend config.json, as in diffusers (e.g. AutoencoderKL's with_encoder=True)
+        model = cls(**{**{k: v for k, v in raw.items() if not k.startswith("_")}, **kw})
         st = os.path.join(path, "diffusion_pytorch_model.safetensors")
         if os.path.exists(st):
             from safetensors.torch import load_file
@@ -427,20 +428,68 @@ class DecoderOutput:  # diffusers/models/vae.py:27-36
         return (self.sample,)[i]
 
 
-class AutoencoderKL(_B200Module):
-    """Decoder half of diffusers' AutoencoderKL (models/autoencoder_kl.py) for the pipeline's `decode_latents`
-    (pipeline_bev_controlnet.py:100-112): same constructor kwargs and checkpoint key names (`decoder.*`,
-    `post_quant_conv.*`; `encoder.*` / `quant_conv.*` of a full checkpoint are accepted and ignored), `.config.scaling_factor`
-    and `.config.block_out_channels` as the pipeline reads them (pipeline_controlnet.py:130-179), `decode(z).sample`.
-    Encoding is not on the path and raises."""
+class DiagonalGaussianDistribution:
+    """diffusers/models/vae.py:397-416 over NCHW `parameters` (mean | logvar along the channels): `.mean`, `.logvar`
+    (clamped to [-30, 20]), `.std`, `.var`, `.sample(generator)` = mean + std * randn_tensor(mean.shape), `.mode()`."""
 
-    def __init__(self, **kwargs):
+    def __init__(self, parameters: torch.Tensor, deterministic: bool = False):
+        self.parameters = parameters
+        self.mean, self.logvar = torch.chunk(parameters, 2, dim=1)
+        self.logvar = torch.clamp(self.logvar, -30.0, 20.0)
+        self.deterministic = deterministic
+        self.std = torch.exp(0.5 * self.logvar)
+        self.var = torch.exp(self.logvar)
+        if deterministic:
+            self.var = self.std = torch.zeros_like(self.mean)
+
+    def sample(self, generator: Optional[torch.Generator] = None) -> torch.Tensor:
+        noise = randn_tensor(self.mean.shape, generator, self.parameters.device, self.parameters.dtype)
+        return self.mean + self.std * noise
+
+    def mode(self) -> torch.Tensor:
+        return self.mean
+
+
+def randn_tensor(shape, generator: Optional[torch.Generator], device, dtype=F32) -> torch.Tensor:
+    """diffusers.utils.torch_utils.randn_tensor for one generator: drawn on the generator's device (a CPU generator
+    feeding a CUDA tensor draws on the host and copies), so a seeded generator gives diffusers' draw."""
+    device = torch.device(device)
+    gen_dev = generator.device if generator is not None else device
+    x = torch.randn(tuple(shape), generator=generator, device=gen_dev, dtype=dtype)
+    return x.to(device)
+
+
+@dataclass
+class AutoencoderKLOutput:  # diffusers/models/autoencoder_kl.py:28-37
+    latent_dist: DiagonalGaussianDistribution
+
+    def __getitem__(self, i):
+        return (self.latent_dist,)[i]
+
+
+class AutoencoderKL(_B200Module):
+    """diffusers' AutoencoderKL (models/autoencoder_kl.py) for the pipeline's `decode_latents` (pipeline_bev_controlnet.py:
+    100-112) and, with `with_encoder=True`, for `encode` (the given-view demo's latents, demo/run_cond_on_view.py:80-86):
+    same constructor kwargs and checkpoint key names, `.config.scaling_factor` and `.config.block_out_channels` as the
+    pipeline reads them (pipeline_controlnet.py:130-179), `decode(z).sample`, `encode(x).latent_dist`.
+    By default the module is the decoder half only (`decoder.*`, `post_quant_conv.*`; `encoder.*` / `quant_conv.*` of a
+    full checkpoint are accepted and ignored) and `encode` raises.  `with_encoder=True` (kept in `.config`, so a saved
+    config.json restores it) holds the full key set, loads it strictly and runs the encoder on the GPU too."""
+
+    def __init__(self, with_encoder: bool = False, **kwargs):
         super().__init__()
         known, extra = _pick(arch.VaeConfig, dict(kwargs))
         cfg = arch.VaeConfig(**{k: (tuple(v) if isinstance(v, list) else v) for k, v in known.items()})
         if cfg.act_fn != "silu" or any(t != "UpDecoderBlock2D" for t in cfg.up_block_types):
             raise ValueError("only the SD-1.5 AutoencoderKL layout (UpDecoderBlock2D, silu) is implemented")
-        self._init_common(cfg, arch.vae_decoder_param_shapes(cfg), extra)
+        self.with_encoder = bool(with_encoder)
+        shapes = arch.vae_decoder_param_shapes(cfg)
+        if self.with_encoder:
+            if any(t != "DownEncoderBlock2D" for t in cfg.down_block_types):
+                raise ValueError("only the SD-1.5 AutoencoderKL encoder layout (DownEncoderBlock2D, silu) is implemented")
+            extra["with_encoder"] = True
+            shapes = OrderedDict(list(arch.vae_encoder_param_shapes(cfg).items()) + list(shapes.items()))
+        self._init_common(cfg, shapes, extra)
         self.training = False
 
     _OLD_ATTN = {"query": "to_q", "key": "to_k", "value": "to_v", "proj_attn": "to_out.0"}  # pre-0.17 checkpoint names
@@ -448,7 +497,7 @@ class AutoencoderKL(_B200Module):
     def load_state_dict(self, state_dict, strict=True, **kw):
         sd = {}
         for k, v in state_dict.items():
-            if k.startswith(("encoder.", "quant_conv.")):
+            if not self.with_encoder and k.startswith(("encoder.", "quant_conv.")):
                 continue
             parts = k.split(".")
             if "attentions" in parts and parts[-2] in self._OLD_ATTN:  # attention_processor.py:_from_deprecated_attn_block
@@ -456,18 +505,77 @@ class AutoencoderKL(_B200Module):
             sd[k] = v
         return super().load_state_dict(sd, strict=strict, **kw)
 
-    use_cuda_graph = True  # decode_latents replays one captured graph per shape
+    use_cuda_graph = True  # decode_latents / encode_latents replay one captured graph per shape
     _decode_graphs: dict = {}
+    _encode_graphs: dict = {}
 
     def engine(self) -> VaeDecoderEngine:
-        eng = self._get_engine(VaeDecoderEngine)
+        """The decoder engine, or with_encoder the VaeEncoderEngine that also decodes (one packed-weight cache)."""
+        eng = self._get_engine(VaeEncoderEngine if self.with_encoder else VaeDecoderEngine)
         if getattr(self, "_graphs_for", None) is not eng:  # weights changed -> engine rebuilt -> graphs stale
-            self._decode_graphs, self._graphs_for = {}, eng
+            self._decode_graphs, self._encode_graphs, self._graphs_for = {}, {}, eng
         return eng
 
-    def encode(self, *a, **k):
-        raise NotImplementedError("AutoencoderKL.encode is not on the generation path (SURVEY.md §2.1); only decode is built")
+    def _encoder_engine(self, x: torch.Tensor) -> VaeEncoderEngine:
+        if not self.with_encoder:
+            raise NotImplementedError("this AutoencoderKL holds the decoder only; build it with with_encoder=True "
+                                      "(AutoencoderKL(..., with_encoder=True) or from_pretrained(..., with_encoder=True)) to encode")
+        if x.shape[-3] != self.arch_cfg.in_channels or x.shape[-2] % 8 or x.shape[-1] % 8:
+            raise ValueError(f"encode expects (..., {self.arch_cfg.in_channels}, H, W) images with H and W divisible by 8, "
+                             f"got {tuple(x.shape)}")
+        return self.engine()
 
+    @torch.no_grad()
+    def encode(self, x: torch.Tensor, return_dict: bool = True):
+        """AutoencoderKL.encode (autoencoder_kl.py:160-171): NCHW images in [-1, 1] -> the posterior over the latents
+        (DiagonalGaussianDistribution of fp32 NCHW (n, 2 * latent_channels, H/8, W/8) moments)."""
+        eng = self._encoder_engine(x)
+        n, _, h, w = x.shape
+        c = self.arch_cfg.latent_channels
+        mom = eng.encode(x.to(self.device))
+        params = mom.view(n, h // 8, w // 8, -1)[..., : 2 * c].permute(0, 3, 1, 2).contiguous()
+        posterior = DiagonalGaussianDistribution(params)
+        return AutoencoderKLOutput(latent_dist=posterior) if return_dict else (posterior,)
+
+    @torch.no_grad()
+    def encode_latents(self, pixel_values: torch.Tensor, sample: bool = False,
+                       generator: Optional[torch.Generator] = None) -> torch.Tensor:
+        """The given-view demo's latents (demo/run_cond_on_view.py:80-86): (b, n_cam, 3, H, W) images in [-1, 1] ->
+        fp32 (b, n_cam, latent_channels, H/8, W/8) = scaling_factor * posterior mean (or, with `sample`, a posterior
+        sample drawn with `generator` like DiagonalGaussianDistribution.sample), on the module's device.  Each shape is
+        one CUDA-graph replay; the sample's noise is drawn outside the graph into a resident buffer."""
+        b, n_cam = pixel_values.shape[:2]
+        x = pixel_values.reshape(b * n_cam, *pixel_values.shape[2:])
+        eng = self._encoder_engine(x)
+        n, _, hh, ww = x.shape
+        h, w, c = hh // 8, ww // 8, self.arch_cfg.latent_channels
+        scale = float(self.config["scaling_factor"])
+        noise = randn_tensor((n, c, h, w), generator, self.device) if sample else None
+
+        def run(xx, nz):
+            return ops.latent_dist(eng.encode(xx), n, h, w, c, noise=nz, scale=scale)
+
+        x = x.to(self.device)
+        if not (self.use_cuda_graph and x.is_cuda):
+            z = run(x, noise)
+        else:
+            key = (id(eng), n, hh, ww, x.dtype, sample)
+            g = self._encode_graphs.get(key)
+            if g is None:
+                xin, nin = x.clone(), (noise.clone() if sample else None)
+                run(xin, nin)  # eager once: sizes the scratch and the split-K workspace
+                torch.cuda.synchronize()
+                graph = torch.cuda.CUDAGraph()
+                with torch.cuda.graph(graph):
+                    out = run(xin, nin)
+                g = self._encode_graphs[key] = (graph, xin, nin, out)
+            graph, xin, nin, out = g
+            xin.copy_(x)
+            if sample:
+                nin.copy_(noise)
+            graph.replay()
+            z = out.clone()
+        return z.reshape(b, n_cam, c, h, w)
     @torch.no_grad()
     def decode(self, z: torch.Tensor, return_dict: bool = True):
         """z: (n, 4, h, w) latents already divided by scaling_factor, as the pipeline passes them -> (n, 3, 8h, 8w)."""

@@ -427,6 +427,37 @@ def pin_views(dst, a, b, coef, view_mask, rows_per_view: int, c: int = 4):
     return dst
 
 
+def pack_image_patches(x):
+    """NCHW images [n, cin, h, w] fp32/bf16 -> bf16 [n*h*w, 64]: the zero-padded 3x3 neighbourhood of every pixel in
+    column order (tap, channel), columns >= 9*cin zero (the A operand of the VAE encoder's conv_in as a K = 64 GEMM)."""
+    global _launches
+    _need_cuda(x)
+    n, cin, h, w = x.shape
+    x = x.contiguous()
+    if x.dtype not in (F32, BF16):
+        x = x.float()
+    out = torch.empty((n * h * w, 64), dtype=BF16, device=x.device)
+    check(_lib.lib().mdb_pack_image_patches(_ptr(x), int(x.dtype == F32), n, cin, h, w, _ptr(out), _stream()),
+          "mdb_pack_image_patches")
+    _launches += 1
+    return out
+
+
+def latent_dist(moments, n: int, h: int, w: int, c: int = 4, noise=None, scale: float = 1.0):
+    """fp32 NHWC moments [n*h*w, >= 2c] (mean | logvar) -> fp32 NCHW [n, c, h, w] =
+    scale * (mean + exp(0.5 * clamp(logvar, -30, 20)) * noise); noise fp32 NCHW or None (scale * mean)."""
+    global _launches
+    _need_cuda(moments, noise)
+    assert moments.dtype == F32 and moments.shape[0] == n * h * w
+    if noise is not None:
+        assert noise.dtype == F32 and noise.is_contiguous() and noise.numel() == n * c * h * w
+    out = torch.empty((n, c, h, w), dtype=F32, device=moments.device)
+    check(_lib.lib().mdb_latent_dist(_ptr(moments), moments.stride(0), n, c, h, w, _ptr(noise), float(scale), _ptr(out),
+                                     _stream()), "mdb_latent_dist")
+    _launches += 1
+    return out
+
+
 def pack_latents(x, cpad: int = 64, repeat: int = 1):
     """[pix, cin] fp32/bf16 -> bf16 [repeat*pix, cpad] zero-padded channels."""
     global _launches

@@ -388,7 +388,9 @@ class BEVControlNetDenoiser:
                 raise ValueError("conditional_latents must be a list[scenes] of list[n_cam] of (4, h, w) tensors or None")
             pin_mode = "change" if conditional_latents_change_every_input else "once"
             pin_mask = torch.tensor([int(c is not None) for row in conditional_latents for c in row], dtype=torch.int32)
-            pin_cond = torch.stack([torch.zeros(c, h, w) if x is None else x.to("cpu", F32)
+            # staged where the given latents already are (AutoencoderKL.encode_latents leaves them on the GPU)
+            pdev = next(x for row in conditional_latents for x in row if x is not None).device
+            pin_cond = torch.stack([torch.zeros(c, h, w, device=pdev) if x is None else x.to(pdev, F32)
                                     for row in conditional_latents for x in row])
             pin_cond = pin_cond.permute(0, 2, 3, 1).contiguous().view(-1, c)
         inputs = dict(camera=camera_param, text=text, image=image, latents=lat_nhwc)
